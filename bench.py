@@ -16,6 +16,9 @@ Reported (one JSON line on stdout, rank 0):
   roofline   the dominant kernel (reweight_lfm) against the measured HBM copy peak
   cpu_baseline  the CPU oracle (a port of the reference pipeline; the reference itself needs
              Eigen/Sophus/range-v3, absent here) on the host cores, bounded sample, same workload
+
+--dump-outputs DIR writes what the last timed step returned (pose estimate, weight sum) and the particle set it left
+behind as DIR/<name>.npy (float64), so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -32,6 +35,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is written into it
 # The CPU reference runs OpenMP teams on a CPU quota (cgroup): spinning idle threads burn the quota and get the
 # whole process throttled (8 threads on 20k particles: 264 ms/step spinning, 33 ms/step sleeping).  Must be set
 # before libgomp initialises.
@@ -42,6 +46,9 @@ UNIT = "steps/s"
 MOTION = (0.1, 0.05, 0.1, 0.05)  # likelihood_params.yaml:6-12
 LFM = dict(max_obstacle_distance=2.0, max_laser_distance=100.0, z_hit=0.5, z_random=0.5, sigma_hit=0.2)  # :55-65
 PATH_STEPS = 100
+# --dump-outputs: at most this many particles (32 B state + 8 B weight each: 40 MB), a seeded sample beyond it
+DUMP_MAX_PARTICLES = 1_000_000
+DUMP_SAMPLE_SEED = 0
 SCALING = "strong"  # the metric is quoted "at 1M particles": N GPUs shard the SAME filter (--weak: --particles per GPU instead)
 
 
@@ -61,7 +68,25 @@ def parse_args():
     ap.add_argument("--grid", type=int, default=2000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-weak-line", action="store_true", help="N > 1: skip the extra weak-scaling measurement (--particles per GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (native arm; "
+                    "with N > 1 the particles are rank 0's shard)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native arm")
+    return args
+
+
+def dump_outputs(out_dir, outputs, states, weights):
+    """outputs: name -> float64 array of the last timed step; states/weights: the particle set after it (a fixed, seeded
+    sample of DUMP_MAX_PARTICLES particles, in index order, when the set is larger)."""
+    if len(weights) > DUMP_MAX_PARTICLES:
+        keep = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(len(weights), DUMP_MAX_PARTICLES, replace=False))
+        states, weights = states[keep], weights[keep]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in {**outputs, "particle_states": states, "particle_weights": weights}.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def make_workload(args):
@@ -297,10 +322,11 @@ def run_native(args):
             dist.barrier()
             torch.cuda.synchronize()
 
-    def measure(n_total, with_clocks):
+    def measure(n_total, with_clocks, keep_outputs=False):
         """K timed steps of ONE filter of n_total particles over `world` GPUs.  Device time: CUDA events on the filter's
         own stream from the first kernel of the step to the read-back (exchanges and the waits inside them included);
-        end to end: host clock around the public update call.  Max over ranks."""
+        end to end: host clock around the public update call.  Max over ranks.  keep_outputs: also return what the
+        last step returned and the particle set it left."""
         shard = n_total // world
         if shard * world != n_total:
             raise SystemExit(f"bench.py: {n_total} particles do not split into {world} equal shards")
@@ -312,7 +338,8 @@ def run_native(args):
             def step(k):
                 r = amcl.update(poses[k], scans[k])  # bb200_amcl_update: synchronous, the estimate is read back inside
                 assert r.updated == 1 and r.resampled == 1
-                return np.array(r.estimate.mean)
+                return {"estimate_mean": np.array(r.estimate.mean), "estimate_cov": np.array(r.estimate.cov).reshape(3, 3),
+                        "weight_sum": np.array([r.weight_sum])}
         else:
             # ONE filter sharded over the ranks.  Each rank calls bb200_amcl_update on its shard; the exchanges (largest
             # weight, fixed-point totals, moments) and the redistribution of resampled states run over NVLink peer memory
@@ -326,7 +353,7 @@ def run_native(args):
             def step(k):
                 out = amcl.update(poses[k], scans[k])
                 assert out is not None and out[2]["resampled"]
-                return out[0]
+                return {"estimate_mean": np.asarray(out[0]), "estimate_cov": np.asarray(out[1]), "weight_sum": np.array([out[2]["weight_sum"]])}
 
         amcl.update_map(bb.SENSOR_LIKELIHOOD_FIELD, lfm, grid)
         amcl.initialize(scenario.initial_mean, scenario.initial_cov)
@@ -355,43 +382,45 @@ def run_native(args):
         def e2e_loop():
             """End to end: host clock around the public update call (host scan in, estimate out), the next K steps of the
             path, without the per-kernel event marks of the loop above."""
-            mean = None
+            outputs = None
             filt.set_timing(False)
             for k in range(args.warmup + args.steps, args.warmup + 2 * args.steps):
                 flush.zero_()
                 sync_all()
                 t0 = time.perf_counter()
-                mean = step(k)
+                outputs = step(k)
                 wall_ms.append((time.perf_counter() - t0) * 1e3)
             sync_all()
-            return mean
+            return outputs
 
         if with_clocks:
             with ClockSampler(local_rank) as clocks:
                 timed_loop()
                 launches = filt.launch_count() - launches0
-                mean = e2e_loop()
+                outputs = e2e_loop()
             clock_summary = clocks.summary()
         else:
             timed_loop()
             launches = filt.launch_count() - launches0
-            mean = e2e_loop()
+            outputs = e2e_loop()
             clock_summary = None
+        particles = filt.particles() if keep_outputs else None
         totals = torch.tensor([sum(device_ms), sum(wall_ms)], dtype=torch.float64, device="cuda")
         if world > 1:
             dist.all_reduce(totals, op=dist.ReduceOp.MAX)
         dev_total_ms, wall_total_ms = totals.tolist()
         last = (args.warmup + 2 * args.steps - 1) % PATH_STEPS
+        mean = outputs["estimate_mean"]
         err = float(np.hypot(mean[2] - scenario.poses[last][0], mean[3] - scenario.poses[last][1]))
         if world > 1:
             amcl.close()
         del amcl
         return {"n_total": n_total, "shard": shard, "dev_ms": dev_total_ms / args.steps, "wall_ms": wall_total_ms / args.steps,
                 "kernels_ms": {name: float(np.mean(v)) for name, v in kernel_ms.items()}, "launches": int(launches), "clocks": clock_summary,
-                "final_position_error_m": err}
+                "final_position_error_m": err, "outputs": outputs, "particles": particles}
 
     n_total = reference_particles(args)
-    m = measure(n_total, with_clocks=True)
+    m = measure(n_total, with_clocks=True, keep_outputs=bool(args.dump_outputs))
     weak = None
     if world > 1 and not args.weak and not args.no_weak_line:
         weak = measure(args.particles * world, with_clocks=False)  # the same run at --particles PER GPU
@@ -440,6 +469,8 @@ def run_native(args):
                             "roofline_frac": wbytes / (wk1 * 1e-3) / 1e9 / peak, "final_position_error_m": weak["final_position_error_m"]}
         if not args.no_cpu_baseline and world == 1:  # timed beside the GPU arm on rank 0 at N = 1 only
             line["cpu_baseline"] = cpu_reference_steps_per_s(args, scenario, n_total, steps=5)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, m["outputs"], *m["particles"])
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

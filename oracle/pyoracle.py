@@ -5,9 +5,12 @@ legs only.  The product package (beluga_b200/) never imports this module.
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -28,37 +31,19 @@ def build(force: bool = False) -> str:
     return _LIB_PATH
 
 
-def _cpu_stamp() -> str:
-    """Identifies the host CPU: a -march=native build must not run on another machine."""
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("flags"):
-                import hashlib
-
-                return hashlib.sha1(line.encode()).hexdigest()[:16]
-    except OSError:
-        pass
-    return "unknown"
-
-
 def use_native_build() -> bool:
     """Timing legs only (bench.py): switch to a -march=native build of the same sources, compiled on this machine
-    (make native).  Must run before the first oracle call.  Returns False (and keeps the portable build) if the
+    (make native) into a temporary directory that is removed at exit, so that a timing run writes nothing into the
+    source tree.  Must run before the first oracle call.  Returns False (and keeps the portable build) if the
     library is already loaded or the build fails."""
     global _LIB_PATH
     if _lib is not None:
         return False
-    native = os.path.join(_HERE, "_build", "native", "liboracle.so")
-    stamp_path = native + ".cpu"
-    stamp = _cpu_stamp()
-    srcs = [os.path.join(_HERE, f) for f in _SOURCES]
-    fresh = (os.path.exists(native) and os.path.exists(stamp_path) and open(stamp_path).read() == stamp and
-             all(os.path.getmtime(s) <= os.path.getmtime(native) for s in srcs))
-    if not fresh:
-        if subprocess.run(["make", "-C", _HERE, "-s", "-B", "native"]).returncode != 0:
-            return False
-        with open(stamp_path, "w") as f:
-            f.write(stamp)
+    out_dir = tempfile.mkdtemp(prefix="beluga_b200_oracle_")
+    atexit.register(shutil.rmtree, out_dir, ignore_errors=True)
+    native = os.path.join(out_dir, "liboracle.so")
+    if subprocess.run(["make", "-C", _HERE, "-s", "-B", "native", f"NATIVE_OUT={native}"]).returncode != 0:
+        return False
     _LIB_PATH = native
     globals()["build"] = lambda force=False: native  # lib() must not fall back to rebuilding the portable library
     return True

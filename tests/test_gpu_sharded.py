@@ -23,7 +23,7 @@ def test_two_gpu_shards_match_single_gpu(mode):
 
     bb_build.build()
     if bb.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
            "--master-port", str(29711 + 2 * MODES.index(mode)), os.path.join(ROOT, "tests", "_shard_gpu_worker.py"), "40000", "6", mode]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
@@ -43,7 +43,7 @@ def test_one_process_two_devices_match_single_gpu(mode):
 
     bb_build.build()
     if bb.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     sc = synthetic.make_scenario(grid_size=200, n_beams=181, steps=8)
     n = 60_000
     kw = dict(systematic=dict(resample_scheme=1), multinomial=dict(resample_scheme=0, recovery_probability_override=0.02),
