@@ -1027,6 +1027,7 @@ int Filter::set_likelihood_field_map(const bb200_likelihood_field_param& p, cons
   // Bordered tile layout for the fixed-point kernel.
   field_.use_fixed = 0;
   field_.bordered = nullptr;
+  field_.bordered_biased = nullptr;
   cudaFree(bordered_);
   bordered_ = nullptr;
   if (fixed_lookup_ && g.width + 2 <= kFixedMaxSide && g.height + 2 <= kFixedMaxSide) {
@@ -1046,6 +1047,10 @@ int Filter::set_likelihood_field_map(const bb200_likelihood_field_param& p, cons
     field_.border_pitch = 1u << kx;
     field_.border_x_max = static_cast<uint32_t>(4 * (g.width + 1) + 3);
     field_.border_y_max = static_cast<uint32_t>(g.height + 1);
+    // The kernel adds the biased 32-bit index to this base, so every index of the table plus the bias must stay below 2^32.
+    const uint32_t bias = fixed_index_bias(kx);
+    if (static_cast<uint64_t>(bias) + bordered.size() <= (1ull << 32))
+      field_.bordered_biased = reinterpret_cast<const double*>(reinterpret_cast<uintptr_t>(bordered_) - static_cast<uintptr_t>(bias) * sizeof(double));
     field_.use_fixed = 1;
   }
   field_.tiled = tiled_;

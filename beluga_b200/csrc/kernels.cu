@@ -25,7 +25,7 @@
 #define BB200_RW_THREADS 256
 #endif
 #ifndef BB200_RW_UNROLL
-#define BB200_RW_UNROLL 2
+#define BB200_RW_UNROLL 4
 #endif
 #ifndef BB200_RW_BLOCKS
 #define BB200_RW_BLOCKS 4
@@ -421,7 +421,7 @@ __global__ void __launch_bounds__(256) schedule_scatter_kernel(const uint32_t* _
 
 constexpr int kRwThreads = BB200_RW_THREADS;  // x kRwBlocksPerSm CTAs per SM
 constexpr int kRwBlocksPerSm = BB200_RW_BLOCKS;
-constexpr int kRwUnroll = BB200_RW_UNROLL;  // groups of four beams in flight per thread
+constexpr int kRwUnroll = BB200_RW_UNROLL;  // groups of four beams per trip of the beam loop
 constexpr uint32_t kChunkBeams = 2048; // beams staged per shared-memory chunk (32 KB), multiple of 4
 
 /// floor(g) as int32 for |g| < 2^31: one F2I.F64.FLOOR (saturating).
@@ -571,11 +571,11 @@ __global__ void __launch_bounds__(kRwThreads, kRwBlocksPerSm)
 // coordinate, about once every two steps among a million particles) or a particle out of the 2^13 range
 // redoes its beams with the reference's own operation sequence; nothing else in the loop branches.
 // Out-of-grid end points clamp (one DPX add-min per coordinate, which also strips the bias) to the
-// one-cell border holding the unknown-space value, so the load is unconditional.
+// one-cell border holding the unknown-space value, so the load is unconditional.  A warp whose particles'
+// scans all stay on the bordered map skips the clamp and indexes with the biased words (fixed_lookup_in_map).
 
-constexpr double kFixedMagicX = 393216.0;   // 1.5 * 2^18: ulp 2^-34; high word = 0x41180000 + floor(4 g)    for |g| < 2^17
-constexpr double kFixedMagicY = 1572864.0;  // 1.5 * 2^20: ulp 2^-32; high word = 0x41380000 + floor(g)      for |g| < 2^19
-constexpr uint32_t kFixedBiasX = 0x41180000u, kFixedBiasY = 0x41380000u;
+constexpr double kFixedMagicX = 393216.0;   // 1.5 * 2^18: ulp 2^-34; high word = kFixedBiasX + floor(4 g)    for |g| < 2^17
+constexpr double kFixedMagicY = 1572864.0;  // 1.5 * 2^20: ulp 2^-32; high word = kFixedBiasY + floor(g)      for |g| < 2^19
 // The magic constants ride in the FMAs' addend (per-particle offsets ox, oy below), which saves the two additions per beam
 // but lets THREE roundings at the magic's ulp into the word instead of one (the offset sum and both FMAs): the computed
 // fixed-point value is within 3 half-ulps + 2^-36 cells of the reference's.  Two ulps of guard are added to the offset so
@@ -591,6 +591,7 @@ struct FixedParticle {
   double ox, oy;         // field-frame position in cells, plus the border cell, plus magic constant and guard
   uint32_t x_max, y_max; // 4 (width + 1) + 3, height + 1: largest 4 * padded x (+ 2 fraction bits) and padded y
   uint32_t row_pitch;    // 4 * 2^kx: elements per row of cells (four rows of tiles' worth per tile row)
+  bool in_map;           // every end point of the scan lands in the bordered map: fixed_lookup_in_map applies
 };
 
 /// `margin` collects the smallest fraction word seen (<= kFixedAmbiguous: a coordinate too close to a cell edge to call).
@@ -609,6 +610,21 @@ __device__ __forceinline__ double fixed_lookup(const double* __restrict__ border
   asm("lop3.b32 %0, %1, 3, %2, 0xB8;" : "=r"(low) : "r"(ux), "r"(uy));
   const uint32_t idx = (uy & ~3u) * q.row_pitch + low;
   return __ldg(bordered + idx);
+}
+
+/// fixed_lookup for a particle whose end points all land in the bordered map (q.in_map): no clamp, and no bias stripped.
+/// The biases' low 19 bits are clear, so the bit-select and the mask act on the cell bits as before, and the index is the
+/// bordered index plus fixed_index_bias(kx) (mod 2^32), which `biased` (FieldView::bordered_biased) takes back off.
+__device__ __forceinline__ double fixed_lookup_in_map(const double* __restrict__ biased, const FixedParticle& q, double px, double py,
+                                                      uint32_t& margin) {
+  const double gx = fma(px, q.cx, fma(-py, q.sx, q.ox));
+  const double gy = fma(px, q.sx, fma(py, q.cx, q.oy));
+  margin = __vimin3_u32(margin, static_cast<uint32_t>(__double2loint(gx)), static_cast<uint32_t>(__double2loint(gy)));
+  const uint32_t hx = static_cast<uint32_t>(__double2hiint(gx)), hy = static_cast<uint32_t>(__double2hiint(gy));
+  uint32_t low;
+  asm("lop3.b32 %0, %1, 3, %2, 0xB8;" : "=r"(low) : "r"(hx), "r"(hy));
+  const uint32_t idx = (hy & ~3u) * q.row_pitch + low;
+  return __ldg(biased + idx);
 }
 
 /// The reference's operation sequence (field_lookup) against the bordered layout.
@@ -635,42 +651,54 @@ struct ScanParam {
   double2 p[kParamBeams];
 };
 
-#define BB200_PRAGMA_STR(x) _Pragma(#x)
-#define BB200_PRAGMA_UNROLL(n) BB200_PRAGMA_STR(unroll n)
+// One group of four beams of the pipeline below: look up beams B..B+3, then add the previous group to acc.
+#define BB200_FIXED_STEP(POINT, B, LOOKUP, TABLE)                                                             \
+  {                                                                                                           \
+    const double2 p0 = POINT(B), p1 = POINT((B) + 1), p2 = POINT((B) + 2), p3 = POINT((B) + 3);               \
+    const double g0 = LOOKUP(TABLE, q, p0.x, p0.y, margin);                                                   \
+    const double g1 = LOOKUP(TABLE, q, p1.x, p1.y, margin);                                                   \
+    const double g2 = LOOKUP(TABLE, q, p2.x, p2.y, margin);                                                   \
+    const double g3 = LOOKUP(TABLE, q, p3.x, p3.y, margin);                                                   \
+    acc = acc + ((f0 + f1) + (f2 + f3));                                                                      \
+    f0 = g0, f1 = g1, f2 = g2, f3 = g3;                                                                       \
+  }
 // libstdc++ transform_reduce (numeric:439-462): groups of four, init += ((f0+f1)+(f2+f3)), then one by one.
-#define BB200_FIXED_SUM(POINT, COUNT, LOOKUP, TABLE)                                                                       \
+#define BB200_FIXED_PIPELINE(POINT, COUNT, LOOKUP, TABLE)                                                     \
+  if (4 <= (COUNT)) {                                                                                         \
+    /* Software pipeline: the loads of the next four beams are issued before the previous four are summed */  \
+    /* (a warp issues in order: summing first would leave it with four loads in flight, then none).       */  \
+    double f0, f1, f2, f3;                                                                                    \
+    {                                                                                                         \
+      const double2 p0 = POINT(0), p1 = POINT(1), p2 = POINT(2), p3 = POINT(3);                               \
+      f0 = LOOKUP(TABLE, q, p0.x, p0.y, margin);                                                              \
+      f1 = LOOKUP(TABLE, q, p1.x, p1.y, margin);                                                              \
+      f2 = LOOKUP(TABLE, q, p2.x, p2.y, margin);                                                              \
+      f3 = LOOKUP(TABLE, q, p3.x, p3.y, margin);                                                              \
+    }                                                                                                         \
+    b = 4;                                                                                                    \
+    /* kRwUnroll groups per trip and a single exit test: the loop bookkeeping is one compare and branch per trip */\
+    for (; b + 4 * kRwUnroll <= (COUNT); b += 4 * kRwUnroll) {                                                \
+      _Pragma("unroll") for (uint32_t u = 0; u < 4 * kRwUnroll; u += 4) BB200_FIXED_STEP(POINT, uint64_t{b} + u, LOOKUP, TABLE)\
+    }                                                                                                         \
+    _Pragma("unroll 1") for (; b + 4 <= (COUNT); b += 4) BB200_FIXED_STEP(POINT, b, LOOKUP, TABLE)            \
+    acc = acc + ((f0 + f1) + (f2 + f3));                                                                      \
+  }                                                                                                           \
+  for (; b < (COUNT); ++b) {                                                                                  \
+    const double2 p0 = POINT(b);                                                                              \
+    acc = acc + LOOKUP(TABLE, q, p0.x, p0.y, margin);                                                         \
+  }
+#define BB200_FIXED_SUM(POINT, COUNT)                                                                         \
   do {                                                                                                        \
     const double acc_before = acc;                                                                            \
     uint32_t margin = margin_start;                                                                           \
     uint32_t b = 0;                                                                                           \
-    if (4 <= (COUNT)) {                                                                                       \
-      /* Software pipeline: the loads of the next four beams are issued before the previous four are summed */\
-      /* (a warp issues in order: summing first would leave it with four loads in flight, then none).       */\
-      double f0, f1, f2, f3;                                                                                  \
-      {                                                                                                       \
-        const double2 p0 = POINT(0), p1 = POINT(1), p2 = POINT(2), p3 = POINT(3);                             \
-        f0 = LOOKUP(TABLE, q, p0.x, p0.y, margin);                                                            \
-        f1 = LOOKUP(TABLE, q, p1.x, p1.y, margin);                                                            \
-        f2 = LOOKUP(TABLE, q, p2.x, p2.y, margin);                                                            \
-        f3 = LOOKUP(TABLE, q, p3.x, p3.y, margin);                                                            \
-      }                                                                                                       \
-      b = 4;                                                                                                  \
-      BB200_PRAGMA_UNROLL(BB200_RW_UNROLL) for (; b + 4 <= (COUNT); b += 4) {                                 \
-        const double2 p0 = POINT(b), p1 = POINT(b + 1), p2 = POINT(b + 2), p3 = POINT(b + 3);                 \
-        const double g0 = LOOKUP(TABLE, q, p0.x, p0.y, margin);                                               \
-        const double g1 = LOOKUP(TABLE, q, p1.x, p1.y, margin);                                               \
-        const double g2 = LOOKUP(TABLE, q, p2.x, p2.y, margin);                                               \
-        const double g3 = LOOKUP(TABLE, q, p3.x, p3.y, margin);                                               \
-        acc = acc + ((f0 + f1) + (f2 + f3));                                                                  \
-        f0 = g0, f1 = g1, f2 = g2, f3 = g3;                                                                   \
-      }                                                                                                       \
-      acc = acc + ((f0 + f1) + (f2 + f3));                                                                    \
+    /* One loop per warp: a divergent beam loop loses the uniform datapath for the scan points (take_chunk_ticket). */\
+    if (__all_sync(0xffffffffu, q.in_map)) {                                                                  \
+      BB200_FIXED_PIPELINE(POINT, COUNT, fixed_lookup_in_map, field.bordered_biased);                         \
+    } else {                                                                                                  \
+      BB200_FIXED_PIPELINE(POINT, COUNT, fixed_lookup, field.bordered);                                       \
     }                                                                                                         \
-    for (; b < (COUNT); ++b) {                                                                                \
-      const double2 p0 = POINT(b);                                                                            \
-      acc = acc + LOOKUP(TABLE, q, p0.x, p0.y, margin);                                                       \
-    }                                                                                                         \
-    if (margin <= kFixedAmbiguous) { /* a coordinate within ~2^-30 cells of a cell edge, or a particle out of range */ \
+    if (margin <= kFixedAmbiguous) { /* a coordinate within ~2^-30 cells of a cell edge, or a particle out of range */\
       const Pose2 te = field_frame_pose(field, states, i, active);                                            \
       acc = acc_before;                                                                                       \
       b = 0;                                                                                                  \
@@ -703,6 +731,13 @@ __device__ __forceinline__ void fixed_particle_setup(const FieldView& field, con
   q.x_max = field.border_x_max;
   q.y_max = field.border_y_max;
   q.row_pitch = 4u * field.border_pitch;
+  // In-map test in padded cells: |px*c - py*s| <= (|px| + |py|) max(|c|, |s|) <= points_radius max(|c|, |s|), and the
+  // fixed-point sums are within 2^-30 cells of that, so half a cell of margin keeps every floor in 0 .. side + 1.
+  // False for NaN and for maps whose biased indices would wrap.
+  const double r = points_radius * fmax(fabs(q.cx), fabs(q.sx)) + 0.5;
+  const double gx = t.x * inv + 1.0, gy = t.y * inv + 1.0;
+  q.in_map = field.bordered_biased != nullptr && gx - r >= 0.0 && gx + r <= static_cast<double>(field.width + 2) && gy - r >= 0.0 &&
+             gy + r <= static_cast<double>(field.height + 2);
 }
 
 #if BB200_RW_CHUNK > 0
@@ -771,7 +806,7 @@ __global__ void __launch_bounds__(kRwThreads, kRwBlocksPerSm)
     fixed_particle_setup(field, states, i, active, points_radius, q, margin_start);
     double acc = field.init;
 #define BB200_POINT(k) scan.p[(k)]
-    BB200_FIXED_SUM(BB200_POINT, n_points, fixed_lookup, field.bordered);
+    BB200_FIXED_SUM(BB200_POINT, n_points);
 #undef BB200_POINT
     if (active) {
       const double likelihood = field.exp_epilogue ? exp(acc) : acc;
@@ -839,7 +874,7 @@ __global__ void __launch_bounds__(kRwThreads, kRwBlocksPerSm)
     mbarrier_wait(&s_bar, phase);
     phase ^= 1u;
 #define BB200_POINT(k) s_pts[(k)]
-    BB200_FIXED_SUM(BB200_POINT, count, fixed_lookup, field.bordered);
+    BB200_FIXED_SUM(BB200_POINT, count);
 #undef BB200_POINT
     if (base + kChunkBeams < n_points) __syncthreads();
   }
@@ -852,6 +887,8 @@ __global__ void __launch_bounds__(kRwThreads, kRwBlocksPerSm)
   publish_weight_max(active ? weight_order_bits(w) : 0ull, &s_max, &s_arrived, kRwThreads / kWarp, scalars);
 }
 #undef BB200_FIXED_SUM
+#undef BB200_FIXED_PIPELINE
+#undef BB200_FIXED_STEP
 
 // ---- reweight (beam model; a4 + a5) -----------------------------------------------------------
 // BeamSensorModel (sensor/beam_model.hpp:104-150): one thread per particle, beams in the inner

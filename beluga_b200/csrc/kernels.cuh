@@ -34,6 +34,10 @@ struct FieldView {
   uint32_t border_pitch;  // 2^border_kx
   uint32_t border_x_max;  // 4 (width + 1) + 3: largest 4 * padded x with its two fraction bits
   uint32_t border_y_max;  // height + 1: largest padded y
+  // `bordered` minus fixed_index_bias(border_kx) elements: what the fixed-point kernel indexes with the unclamped, still
+  // biased words of end points that are known to land on the map.  Null when the biased indices of this map would wrap
+  // around 2^32 (every such end point then takes the clamped lookup).
+  const double* bordered_biased;
   int use_fixed;          // launch the fixed-point kernel (map small enough for 16.16 cell coordinates)
 };
 
@@ -43,6 +47,11 @@ BB_HD uint32_t bordered_index(uint32_t px, uint32_t py, int kx) {
 }
 /// Largest padded grid side the fixed-point kernel accepts (cell coordinates below 2^13).
 constexpr int kFixedMaxSide = 8000;
+/// High words of the fixed-point x and y sums with the cell bits zero (see kernels.cu); their low 19 bits are clear.
+constexpr uint32_t kFixedBiasX = 0x41180000u, kFixedBiasY = 0x41380000u;
+/// What the bordered index gains, modulo 2^32, when the fixed-point kernel feeds the raw high words to its index arithmetic
+/// instead of the words minus the biases: (kFixedBiasY * row pitch + kFixedBiasX) mod 2^32, row pitch 4 * 2^kx.
+BB_HD uint32_t fixed_index_bias(int kx) { return kFixedBiasY * (4u << kx) + kFixedBiasX; }
 
 /// Device view of the occupancy grid (beam model).
 struct OccupancyView {
